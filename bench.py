@@ -33,6 +33,8 @@ reference's GeoBench-2D default skips the first 35 schedule steps (`--start-step
             default (fixed convolution shapes, tuned inside the warm-up steps; `--no-cudnn-benchmark` for the A/B).
 `--sweep M`: BASELINE.json configs[2]: M edits sharded i mod W (DistributedSampler order, tail padding included), batches of
             `--edits`, final latents gathered over NCCL inside the timed region; strong scaling, reported as `sweep`.
+`--dump-outputs DIR`: the images the last timed batch returned, DIR/images.npy (float32); the inputs depend only on the
+            arguments (seeded synthetic edits, seeded stand-in weights), so two builds compare output for output.
 """
 from __future__ import annotations
 
@@ -77,7 +79,30 @@ def parse():
     ap.add_argument("--active-frac-steps", type=int, default=4,
                     help="schedule steps of the batch run under CUPTI for gpu_active_frac (4 = quick default; the batch "
                          "boundaries weigh 12x more there than in the full 50-step schedule -- pass 50 for the real figure)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the edited images of the last timed batch to DIR/images.npy "
+                         "(float32, [edits,H,W,3], 0..255; a fixed seeded sample of the pixels beyond 64 MB) so that two "
+                         "builds can be compared output for output on identical inputs")
+    args = ap.parse_args()
+    if args.dump_outputs and args.sweep:
+        ap.error("--dump-outputs applies to the batch benchmark, not to --sweep")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, name, arr):
+    """arr -> out_dir/<name>.npy as float32; above DUMP_BYTES a seeded sample of the flattened values (the same
+    elements for the same shape, so runs with the same arguments stay comparable)."""
+    import numpy as np
+    a = np.asarray(arr, dtype=np.float32)
+    cap = DUMP_BYTES // a.itemsize
+    if a.size > cap:
+        idx = np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))
+        a = a.reshape(-1)[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def peaks():
@@ -421,6 +446,8 @@ def run_ours(args):
     launches = int(sum(counts.values()))
     value = world * E * args.steps / t_dev
     finite = bool(torch.isfinite(out.float()).all().item())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "images" if world == 1 else f"images_rank{rank}", out.cpu().numpy())
 
     # ---- roofline of the dominant kernel + every attention shape of the step, from the event pairs of the timed region
     groups = {}
